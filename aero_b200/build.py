@@ -4,6 +4,7 @@ from __future__ import annotations
 import glob
 import hashlib
 import os
+import shutil
 import subprocess
 import sys
 
@@ -33,7 +34,9 @@ def build(force=False, verbose=False):
     dig = _digest()
     if not force and os.path.exists(LIB) and os.path.exists(stamp) and open(stamp).read() == dig:
         return LIB
-    nvcc = os.environ.get("NVCC", "nvcc")
+    # NVCC, else nvcc on PATH, else the toolkit at CUDA_HOME: the CUDA bin directory is often missing from a plain user's PATH
+    nvcc = os.environ.get("NVCC") or shutil.which("nvcc") or \
+        os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")
     objs = []
     os.makedirs(os.path.join(HERE, "build"), exist_ok=True)
     procs = []

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- audio-seconds/sec of the AERO generator forward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 4-16|12-48|11-44|train]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 4-16|12-48|11-44|train] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward over one batch of synthetic white-noise clips per GPU; clips are independent, so ranks shard
@@ -20,6 +20,8 @@ the batch with no data-path collective ("weak" scaling: the per-GPU batch is fix
              in a separate eager pass of the same K steps; fraction of the measured burst AND sustained cuBLAS bf16 rates.
   step     : whole-step achieved TFLOP/s against the same peaks, and the step time against the sum of its launches' own
              rooflines (tools/traffic_model.py: algorithmic bytes / FLOPs per launch).
+  --dump-outputs DIR : after the timed steps, DIR/out.npy (float32) holds the waveform the last timed step returned on rank 0.
+             Inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
   cpu_baseline / --impl reference : the oracle port (oracle/aero_oracle.py, the same torch library calls the reference
              makes) on the host cores, BASELINE.md section 3 protocol.  The reference is a Python package and cannot travel
              to the GPU box; oracle/ is its pinned restatement.
@@ -249,6 +251,23 @@ def run_reference(args, cfg, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, out):
+    """Write `out` as <path>/out.npy in float32.  Beyond DUMP_MAX_BYTES it is a fixed seeded sample of 4 M flattened
+    positions instead, listed in out_index.npy (float64 holds them exactly)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    flat = out.detach().float().cpu().reshape(-1)
+    if flat.numel() * 4 <= DUMP_MAX_BYTES:
+        np.save(os.path.join(path, "out.npy"), flat.view(out.shape).numpy())
+        return
+    idx = torch.randint(0, flat.numel(), (4 << 20,), generator=torch.Generator().manual_seed(SEED)).sort().values
+    np.save(os.path.join(path, "out.npy"), flat[idx].numpy())
+    np.save(os.path.join(path, "out_index.npy"), idx.double().numpy())
+
+
 def timed_steps(fn, steps, barrier):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
@@ -273,8 +292,14 @@ def main():
     ap.add_argument("--precision", type=int, default=None,
                     help="engine precision: 2 (default) FP16-stored activations / kind::f16 tcgen05, 1 fp32 storage / kind::tf32, "
                          "0 every kernel in exact fp32")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (rank 0) to DIR/out.npy, float32")
     ap.add_argument("--_cpu_probe", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config == "train" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the GPU inference configurations (--impl ours, --config other than train)")
     if args.config == "train":
         import bench_train
         return bench_train.main(args)
@@ -332,7 +357,14 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_dev = timed_steps(lambda: model(x_dev), args.steps, barrier)
+    last = []
+
+    def graph_step():
+        last[:] = [model(x_dev)]
+    ms_dev = timed_steps(graph_step, args.steps, barrier)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0])
+    del last[:]
 
     # ---- the same K steps launched eagerly with CUDA events around the roofline kernel family
     fam = ("decoder.0.rw", "decoder.1.rw", "decoder.2.rw", "decoder.3.rw")      # tags = packed-weight names

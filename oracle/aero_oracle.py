@@ -17,10 +17,9 @@ reference calls is available in two forms:
     an independent statement the CUDA kernels are compared against.
 
 Pinning: the reference ships no tests or golden vectors (SURVEY.md section 4, 8c), so parity is pinned
-against the reference *itself*: ``tests/golden/make_golden.py`` imports ``/root/reference``
-unmodified, runs ``Aero.forward`` on seeded inputs and commits the outputs;
-``tests/test_oracle.py`` checks both forms of this oracle against those vectors (and, when
-``/root/reference`` is present, against the live reference, block by block).
+against the reference *itself*: ``tests/golden/make_golden.py`` imports the reference
+unmodified, runs ``Aero.forward`` and single blocks on seeded inputs and commits the outputs;
+``tests/test_oracle.py`` checks both forms of this oracle against those vectors.
 """
 from __future__ import annotations
 

@@ -1,8 +1,8 @@
 """Generate the golden vectors under tests/golden/ by running the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):
+Run with a checkout of the reference:
 
-    python tests/golden/make_golden.py
+    AERO_REFERENCE=<checkout of the reference> python tests/golden/make_golden.py [case ...]
 
 For every case it (1) seeds torch, builds the reference ``src.models.aero.Aero`` from the
 experiment kwargs, (2) applies ``tests.util.trained_like_`` to its state_dict, (3) runs
@@ -12,9 +12,10 @@ waveform, sub-sampled spectra / block activations and a digest of the weights in
 ``<case>.npz``.  Inputs and weights are *recipes* (seed + rule), not blobs: the consumer
 rebuilds them with the same torch build.  A second file, ``stft_cases.npz``, holds
 ``spectro`` / ``ispectro`` outputs (reference src/models/spec.py) for the window/hop pairs the
-path uses.
+path uses, ``mrstft_cases.npz`` the multi-resolution STFT loss and ``ref_blocks.npz`` single reference blocks
+(``make_blocks``).  Naming cases regenerates only those.
 
-The GPU box has no /root/reference; tests there read only the committed .npz files.
+Tests read only the committed .npz files.
 """
 import os
 import sys
@@ -56,7 +57,7 @@ STFT_CASES = [  # n_fft, hop, win, batch-shape, length
 
 def main():
     ref = import_reference()
-    assert ref is not None, "needs /root/reference"
+    assert ref is not None, "set AERO_REFERENCE to a checkout of the reference"
     torch.set_num_threads(os.cpu_count())
     only = set(sys.argv[1:])
     for name, exp, B, L in CASES:
@@ -123,6 +124,32 @@ def main():
         print("stft case", i, tuple(z.shape), tuple(y.shape))
     np.savez_compressed(os.path.join(HERE, "stft_cases.npz"), **blob)
     make_mrstft(ref)
+    make_blocks(ref)
+
+
+def make_blocks(ref):
+    """One BLSTM and one LocalState block of the reference (encoder 3, DConv layer 0) on a seeded activation, and the whole
+    forward on a short seeded clip, for aero_4-16_512_128: 4096 seeded samples + the rms of each output, and the state_dict's
+    key order and weight digest (tests/test_oracle.py::test_oracle_matches_reference_blocks_golden)."""
+    kw = aero_kwargs("aero_4-16_512_128")
+    torch.manual_seed(SEED)
+    model = ref["aero"].Aero(**kw).eval()
+    model.load_state_dict(trained_like_(model.state_dict()))
+    sd = model.state_dict()
+    h = white_noise((6, 96, 251), seed=5)
+    layer = model.encoder[3].dconv.layers[0]
+    with torch.no_grad():
+        outs = {"lstm": layer["lstm"](h), "time_attn": layer["time_attn"](h), "forward": model(white_noise((1, 1, 5000)))}
+    blob = {"digest": np.float64(weights_digest(sd)), "keys": np.array(list(sd))}
+    for tag, a in outs.items():
+        flat = a.reshape(-1)
+        idx = sample_indices(flat.numel(), 4096)
+        blob[tag + "/shape"] = np.array(a.shape)
+        blob[tag + "/idx"] = idx.numpy().astype(np.int32)
+        blob[tag + "/val"] = flat[idx].numpy()
+        blob[tag + "/rms"] = np.float64(flat.double().pow(2).mean().sqrt())
+        print("block", tag, tuple(a.shape))
+    np.savez_compressed(os.path.join(HERE, "ref_blocks.npz"), **blob)
 
 
 MRSTFT_CASES = [  # batch, length, seed offset, scale of the estimate's perturbation

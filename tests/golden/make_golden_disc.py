@@ -1,7 +1,7 @@
 """Golden vectors for the MelGAN multi-scale discriminator (SURVEY.md section 8f rank 3) from the UNMODIFIED reference
 (`src/models/discriminators.py:57-78`) in fp64:
 
-    python tests/golden/make_golden_disc.py
+    AERO_REFERENCE=<checkout of the reference> python tests/golden/make_golden_disc.py
 
 Weights are a recipe (tests/util.disc_recipe_state: 16.9 M parameters would be 68 MB) plus a digest; stored are sub-sampled feature maps of every layer of every scale for a seeded waveform, and the
 gradients (256 samples + rms per parameter, and the full input gradient) of  loss = sum over all feature maps of mean(feature * R)
@@ -21,7 +21,7 @@ def build_reference():
     import importlib
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "src" or k.startswith("src.")}
     path_saved = list(sys.path)
-    sys.path[:] = ["/root/reference"] + [p for p in sys.path if "repo" not in os.path.abspath(p or ".")]
+    sys.path[:] = [os.environ["AERO_REFERENCE"]] + [p for p in sys.path if os.path.abspath(p or ".") != os.path.dirname(os.path.dirname(HERE))]
     try:
         mod = importlib.import_module("src.models.discriminators")
     finally:

@@ -1,13 +1,13 @@
 """Golden vectors for the TRAINING path: parameter gradients of the UNMODIFIED reference generator under autograd.
 
-    python tests/golden/make_golden_train.py
+    AERO_REFERENCE=<checkout of the reference> python tests/golden/make_golden_train.py
 
 For every case: seed, build the reference ``src.models.aero.Aero``, apply ``tests.util.trained_like_``, switch to
 ``train()`` (batch-statistics BatchNorm in the FTB blocks), run ``out = model(mix)`` on seeded white noise, back-propagate
 the scalar ``loss = sum(out * R) / out.numel()`` (model promoted to fp64: see below) with R a seeded noise tensor (so the gradient of the waveform is R / numel: a
 dense, well-conditioned cotangent), and store, per parameter, the gradient's rms and 256 seeded samples, plus the training-mode
 output (sub-sampled) and the BatchNorm running buffers after the step.  The consumer rebuilds inputs and weights from the same
-recipes.  The GPU box has no /root/reference; tests there read only the committed .npz files."""
+recipes.  Tests read only the committed .npz files."""
 import os
 import sys
 
@@ -34,7 +34,7 @@ def cotangent(shape, seed):
 
 def main():
     ref = import_reference()
-    assert ref is not None, "needs /root/reference"
+    assert ref is not None, "set AERO_REFERENCE to a checkout of the reference"
     torch.set_num_threads(os.cpu_count())
     for name, exp, B, L in CASES:
         kw = aero_kwargs(exp)

@@ -1,6 +1,5 @@
 """Pin the oracle: both forms of oracle/aero_oracle.py against the golden vectors produced by the
-unmodified reference (tests/golden/make_golden.py), and -- where /root/reference exists -- against
-the live reference.  CPU only."""
+unmodified reference (tests/golden/make_golden.py), whole forwards and single blocks.  CPU only."""
 import glob
 import os
 
@@ -8,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from util import SEED, import_reference, rel_l2, trained_like_, weights_digest, white_noise
+from util import SEED, rel_l2, trained_like_, weights_digest, white_noise
 
 from aero_b200 import Aero, aero_kwargs
 from oracle import aero_oracle as O
@@ -102,29 +101,29 @@ def test_stft_golden(golden_dir):
     assert i >= 6
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="live reference only exists in the build container")
-def test_oracle_vs_live_reference_blocks():
-    ref = import_reference()
+def test_oracle_matches_reference_blocks_golden(golden_dir):
+    """One BLSTM and one LocalState block, in both forms, and the whole forward against the reference's own modules
+    (tests/golden/make_golden.py::make_blocks): seeded samples of each output and its rms."""
+    g = np.load(os.path.join(golden_dir, "ref_blocks.npz"))
     kw = aero_kwargs("aero_4-16_512_128")
-    torch.manual_seed(SEED)
-    rmodel = ref["aero"].Aero(**kw).eval()
-    rmodel.load_state_dict(trained_like_(rmodel.state_dict()))
     torch.manual_seed(SEED)
     mine = Aero(**kw).eval()
     mine.load_state_dict(trained_like_(mine.state_dict()))
     sd = mine.state_dict()
-    assert all(torch.equal(sd[k], v) for k, v in rmodel.state_dict().items())
+    assert list(sd) == list(g["keys"])
+    assert weights_digest(sd) == pytest.approx(float(g["digest"]), rel=1e-12)
+
+    def check(tag, a):
+        assert tuple(a.shape) == tuple(int(v) for v in g[tag + "/shape"])
+        flat = a.reshape(-1)
+        assert rel_l2(flat[torch.from_numpy(g[tag + "/idx"].astype(np.int64))], g[tag + "/val"]) < 1e-5, tag
+        assert abs(float(flat.double().pow(2).mean().sqrt()) / float(g[tag + "/rms"]) - 1) < 1e-5, tag
     h = white_noise((6, 96, 251), seed=5)
     with torch.no_grad():
         for explicit in (False, True):
-            a = O.blstm(h, sd, "encoder.3.dconv.layers.0.lstm", explicit=explicit)
-            b = rmodel.encoder[3].dconv.layers[0]["lstm"](h)
-            assert rel_l2(a, b) < 1e-5
-            a = O.local_state(h, sd, "encoder.3.dconv.layers.0.time_attn", explicit=explicit)
-            b = rmodel.encoder[3].dconv.layers[0]["time_attn"](h)
-            assert rel_l2(a, b) < 1e-5
-        mix = white_noise((1, 1, 5000))
-        assert rel_l2(O.aero_forward(sd, mine.geom, mix), rmodel(mix)) < 1e-5
+            check("lstm", O.blstm(h, sd, "encoder.3.dconv.layers.0.lstm", explicit=explicit))
+            check("time_attn", O.local_state(h, sd, "encoder.3.dconv.layers.0.time_attn", explicit=explicit))
+        check("forward", O.aero_forward(sd, mine.geom, white_noise((1, 1, 5000))))
 
 
 def _mrstft_inputs(g, i):

@@ -69,11 +69,11 @@ def rel_l2(a, b):
     return float((a - b).norm() / b.norm().clamp_min(1e-30))
 
 
-def import_reference():
-    """Import the unmodified reference package (only possible where /root/reference exists)."""
+def import_reference(ref_root=os.environ.get("AERO_REFERENCE", "")):
+    """Import the unmodified reference package from a checkout of it at `ref_root` (default: the AERO_REFERENCE
+    environment variable).  Only the golden-vector generators under tests/golden/ use it; returns None without one."""
     import importlib
-    ref_root = "/root/reference"
-    if not os.path.isdir(ref_root):
+    if not ref_root or not os.path.isdir(ref_root):
         return None
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "src" or k.startswith("src.")}
     path_saved = list(sys.path)
