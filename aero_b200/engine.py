@@ -176,7 +176,8 @@ class AeroEngine:
 
     def _weights_version(self):
         """Cheap change detector for the model's tensors: in-place updates (optimizer steps, load_state_dict) bump
-        `_version`, which only ever grows, so the sum changes whenever any tensor does.  The tensor list is cached;
+        `_version`, which only ever grows, so the sum changes whenever any tensor does.  An update that writes through raw
+        pointers must bump it itself, as aero_b200.optim.FusedAdam.step does.  The tensor list is cached;
         `Aero._apply` / `load_state_dict` (device moves, re-materialised parameters) call invalidate()."""
         if self._plist is None:
             self._plist = list(self.model.parameters()) + list(self.model.buffers())

@@ -1,10 +1,13 @@
-"""Host-side logic of the training engine that needs no GPU: the zeroed-accumulator pool, the operand-split preconditions and the
-arithmetic claim behind the 3xTF32 mode (aero_b200/train_engine.py, include/aero_b200.h aero_split_tf32)."""
+"""Host-side logic of the training engine that needs no GPU: the zeroed-accumulator pool, the operand-split preconditions, the
+arithmetic claim behind the 3xTF32 mode (aero_b200/train_engine.py, include/aero_b200.h aero_split_tf32) and FusedAdam's
+param-group options (aero_b200/optim.py)."""
 import numpy as np
+import pytest
 import torch
 
 from aero_b200 import Aero, aero_kwargs, cabi
 from aero_b200.engine import tf32_round
+from aero_b200.optim import FusedAdam
 from aero_b200.train_engine import TrainEngine
 
 
@@ -66,3 +69,20 @@ def test_three_tf32_products_reproduce_the_fp32_product():
     # device-side rounding (cvt.rna.tf32: ties away) == the host helper used for the goldens
     x = torch.tensor([1.0 + 2.0 ** -11, 1.0 + 2.0 ** -11 + 2.0 ** -20, -(1.0 + 2.0 ** -11)])
     assert np.allclose(tf32_round(x).numpy(), [1.0 + 2.0 ** -10, 1.0 + 2.0 ** -10, -(1.0 + 2.0 ** -10)])
+
+
+def test_fused_adam_state_dict_steps_torch_adam():
+    """A checkpoint of the fast trainer's optimizer resumes under torch.optim.Adam: its param groups carry every option
+    torch.optim.Adam.step reads (no KeyError on the first step).  The options FusedAdam does not implement are refused."""
+    p = torch.ones(3, requires_grad=True)
+    sd = FusedAdam([p], lr=1e-2).state_dict()
+    assert {"weight_decay": 0, "amsgrad": False, "maximize": False}.items() <= sd["param_groups"][0].items()
+    q = torch.ones(3, requires_grad=True)
+    ref = torch.optim.Adam([q])
+    ref.load_state_dict(sd)
+    q.grad = torch.tensor([1.0, -2.0, 0.0])
+    ref.step()
+    assert torch.allclose(q.detach(), torch.tensor([0.99, 1.01, 1.0]))
+    for bad in (dict(weight_decay=1e-4), dict(amsgrad=True), dict(maximize=True)):
+        with pytest.raises(ValueError):
+            FusedAdam([p], **bad)
